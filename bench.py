@@ -5,6 +5,7 @@ north-star multi-GPU metric (SMC-ABC on MA2, N = 1e6, strong scaling) as the `sm
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA, sm_100a)
     python bench.py --impl reference --gpus N ...            # CPU arm: the UNMODIFIED reference
+    python bench.py ... --dump-outputs DIR                   # + what the last timed step returned
 
 One "step" = one batch through the hot path exactly as `Rejection(d, batch_size=1e6)` runs it
 (SURVEY.md section 8d, config 2; elfi/model/utils.py:37-52, samplers.py:140-237):
@@ -30,8 +31,10 @@ data-path collective; the collective path is what `smc_ma2` measures.
 import argparse
 import json
 import os
+import socket
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 import zlib
@@ -50,6 +53,11 @@ WORKLOAD = 'rejection_dist_thr_merge_B1e6_D128_f64'
 # committed ncu --set full capture (1.024039 GB + 11.09 MB); algorithmic bytes are 1.032 GB
 NCU_DRAM_BYTES_PER_LAUNCH = 1.0351e9
 SMC = dict(population=1_000_000, populations=5, quantile=0.5, batch=125_000, seed=1)
+# the reference arm's full result, which our arm quotes when it runs later on the same host: kept
+# per user, stamped with host and time, quoted only from this host and for REFERENCE_MAX_AGE_S
+REFERENCE_LAST = os.path.join(tempfile.gettempdir(), 'elfi_b200_bench_{}'.format(os.getuid()),
+                              'reference_last.json')
+REFERENCE_MAX_AGE_S = 24 * 3600
 
 
 def peaks():
@@ -160,7 +168,7 @@ def dist_env():
 
 # ------------------------------------------------------------------------------ reference arm
 def run_reference(args):
-    """The unmodified reference (baseline/_ref mirror of /root/reference/elfi through
+    """The unmodified reference (oracle/_ref copy or ELFI_REFERENCE checkout, imported through
     oracle/ref_shim.py) on the host cores: its Distance operation on all cores + its
     Rejection.update merge, pipelined like its own batch loop (oracle/ref_arm.py)."""
     rank, local, world = dist_env()
@@ -241,8 +249,10 @@ def run_reference(args):
     }
     if not args.brief:      # lets our arm quote the reference's MA2 pipeline rate of the same box
         try:
-            with open(os.path.join(ROOT, 'gpurun_out', 'bench_reference_last.json'), 'w') as f:
-                json.dump(line, f)
+            os.makedirs(os.path.dirname(REFERENCE_LAST), mode=0o700, exist_ok=True)
+            with open(REFERENCE_LAST, 'w') as f:
+                json.dump({'host': socket.gethostname(), 'written_unix': time.time(),
+                           'line': line}, f)
         except OSError:
             pass
     print(json.dumps(line), flush=True)
@@ -251,6 +261,12 @@ def run_reference(args):
 def cpu_baseline_subprocess():
     """Rank 0, N = 1: the reference arm as a bounded subprocess (a fresh process: its worker pool
     is forked before anything touches CUDA)."""
+    sys.path.insert(0, os.path.join(ROOT, 'oracle'))
+    import ref_shim
+    if not ref_shim.reference_available():
+        return {'value': None, 'unit': 'accepted particles/s', 'cores': os.cpu_count(),
+                'kind': 'reference',
+                'sample': 'not run: the reference ELFI package is not present'}
     try:
         out = subprocess.run([sys.executable, os.path.abspath(__file__), '--impl', 'reference',
                               '--steps', '5', '--warmup', '1', '--brief'],
@@ -483,6 +499,14 @@ def bolfi_config4_block():
             'speedup_fit': cpu_fit * 1e3 / fit_ms, 'speedup_grid': cpu_grid * 1e3 / grid_ms}
 
 
+def dump_outputs(directory, arrays):
+    """DIR/<name>.npy in float64 (the accepted indices are exact in it): the best-n rows (d, t1, t2)
+    the timed region returns, and the last step's distances and accepted row indices (8 MB)."""
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(directory, name + '.npy'), t.double().cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -553,6 +577,10 @@ def run_ours(args):
     barrier()
     ms_total = e0.elapsed_time(e1)
     assert dropped == 0 and count == args.steps * int(n_acc.item())
+    if args.dump_outputs and rank == 0:     # before the untimed runs below reuse the buffers
+        dump_outputs(args.dump_outputs, {
+            'best_d': best[:, 0], 'best_t1': best[:, 1], 'best_t2': best[:, 2],
+            'distances': d, 'accepted_index': idx[:int(n_acc.item())]})
     # dominant kernel alone (distance + mask), per launch, CUDA events on the launch stream
     kev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
            for _ in range(args.steps)]
@@ -646,13 +674,16 @@ def run_ours(args):
            'ms_per_batch': api_dt / api_batches * 1e3, 'runs_s': [round(t, 4) for t in api_times],
            'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': int(api_res.n_samples) * 3 * 8,
            'posterior_mean_t1': api_mean}
-    ref_path = os.path.join(ROOT, 'gpurun_out', 'bench_reference_last.json')
-    if os.path.exists(ref_path):
+    if os.path.exists(REFERENCE_LAST):
         try:
-            with open(ref_path) as f:
-                ref_api = json.load(f)['reference_detail'].get('ma2_rejection_api')
-            if ref_api and 'simulated_per_s' in ref_api:
-                api['reference_arm_same_box'] = ref_api
+            with open(REFERENCE_LAST) as f:
+                saved = json.load(f)
+            age = time.time() - float(saved['written_unix'])
+            ref_api = saved['line']['reference_detail'].get('ma2_rejection_api')
+            if saved['host'] == socket.gethostname() and 0 <= age <= REFERENCE_MAX_AGE_S and \
+                    os.stat(REFERENCE_LAST).st_uid == os.getuid() and \
+                    ref_api and 'simulated_per_s' in ref_api:
+                api['reference_arm_same_box'] = dict(ref_api, age_s=round(age, 1))
                 api['vs_reference_arm'] = api['simulated_particles_per_s'] / \
                     ref_api['simulated_per_s']
         except Exception:
@@ -723,15 +754,15 @@ def main():
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--brief', action='store_true',
                     help='reference arm: only the headline step (used for cpu_baseline)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step returned to DIR/<name>.npy (rank 0)')
     args = ap.parse_args()
-    os.makedirs(os.path.join(ROOT, 'gpurun_out'), exist_ok=True)
     # make sure the in-tree CUDA library and the oracle are built (no-op when up to date); with
     # torchrun only local rank 0 builds, the others wait for the files
     import __graft_entry__ as entry
     if int(os.environ.get('LOCAL_RANK', '0')) == 0:
         entry.build_cuda()
         entry.build_oracle()
-        entry.build_reference()
     else:
         t_wait = time.time() + 600
         while not os.path.exists(entry.LIB) and time.time() < t_wait:

@@ -1,8 +1,8 @@
 """CPU arm of bench.py (`--impl reference`): the UNMODIFIED reference's own code, timed on the host.
 
 BASELINE INFRASTRUCTURE ONLY (like the rest of oracle/): imported by bench.py's reference arm and
-by tests; never by the product.  The reference package is imported through ref_shim (from
-/root/reference in the build container, from the mirror baseline/_ref on the GPU box).
+by tests; never by the product.  The reference package is imported through ref_shim (from the
+checkout that ELFI_REFERENCE points to).
 
 Config #2 step = one 1e6 x 128 batch through the reference's distance node and its rejection
 merge, i.e. exactly what `elfi.Rejection(d, batch_size=1e6)` does per batch:

@@ -1,5 +1,8 @@
-"""Import the UNMODIFIED reference (elfi-dev/elfi): from /root/reference in the build container,
-else from the mirror baseline/_ref/ that __graft_entry__.build_reference() makes for the GPU box.
+"""Import the UNMODIFIED reference (elfi-dev/elfi v0.8.7): from the checkout that the environment
+variable ELFI_REFERENCE points to (the directory holding its `elfi/` package) if it is set, else
+from the copy in oracle/_ref/ that `make -C oracle` (run by __graft_entry__.build()) makes when a
+checkout is present.  It is not part of this repository; without it the reference-driven tests
+skip and the committed goldens stand in.
 
 TEST / BASELINE INFRASTRUCTURE ONLY.  Used by tests/golden/gen_golden*.py to produce the
 committed golden fixtures, by the reference-driven plugin tests and by ``bench.py --impl
@@ -17,8 +20,8 @@ import numpy as np
 
 import os
 
-_MIRROR = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'baseline', '_ref')
-REFERENCE_ROOT = '/root/reference' if os.path.isdir('/root/reference/elfi') else _MIRROR
+REFERENCE_ROOT = os.path.abspath(os.environ['ELFI_REFERENCE']) if os.environ.get('ELFI_REFERENCE') \
+    else os.path.join(os.path.dirname(os.path.abspath(__file__)), '_ref')
 
 
 def reference_available():
@@ -27,6 +30,9 @@ def reference_available():
 
 def import_reference():
     """Return the reference `elfi` module (import it on first call)."""
+    if not reference_available():
+        raise ImportError('the reference ELFI package was not found in {}: build with a checkout '
+                          'of elfi-dev/elfi present, or set ELFI_REFERENCE'.format(REFERENCE_ROOT))
     if 'elfi' in sys.modules and getattr(sys.modules['elfi'], '__file__', '').startswith(
             REFERENCE_ROOT):
         return sys.modules['elfi']

@@ -1,8 +1,8 @@
-"""Generate the golden fixtures from the UNMODIFIED reference (/root/reference).
+"""Generate the golden fixtures from the UNMODIFIED reference (elfi-dev/elfi v0.8.7).
 
-Run in the build container only (the reference is not present on the GPU box):
+Needs a checkout of the reference, which the tests themselves never do:
 
-    python tests/golden/gen_golden.py
+    ELFI_REFERENCE=<checkout of elfi-dev/elfi> python tests/golden/gen_golden.py
 
 Writes tests/golden/*.npz / *.json.  The reference is imported through oracle/ref_shim.py
 (stubs for packages that are absent here and that the sampler path never touches).

@@ -1,6 +1,6 @@
-"""Golden fixtures for the BOLFI sampling path, from the UNMODIFIED reference (/root/reference).
+"""Golden fixtures for the BOLFI sampling path, from the UNMODIFIED reference (elfi-dev/elfi).
 
-    python tests/golden/gen_golden_bolfi.py          (build container only)
+    ELFI_REFERENCE=<checkout of elfi-dev/elfi> python tests/golden/gen_golden_bolfi.py
 
 * mcmc.npz            -- elfi.methods.mcmc.nuts / metropolis chains on analytic targets and the
                          ESS / R-hat of those chains (mcmc.py is pure NumPy).
@@ -20,7 +20,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, os.path.join(ROOT, 'oracle'))
 
-from ref_shim import import_reference  # noqa: E402
+from ref_shim import REFERENCE_ROOT, import_reference  # noqa: E402
 
 elfi = import_reference()
 import elfi_oracle as o  # noqa: E402
@@ -136,7 +136,7 @@ def main():
     # generated in PyStan with Stan's ESS and split R-hat)
     import importlib.util
     spec = importlib.util.spec_from_file_location(
-        'ref_test_mcmc', '/root/reference/tests/unit/test_mcmc.py')
+        'ref_test_mcmc', os.path.join(REFERENCE_ROOT, 'tests', 'unit', 'test_mcmc.py'))
     ref_test = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(ref_test)
     out['stan_chains'] = np.asarray(ref_test.chains_Stan)
