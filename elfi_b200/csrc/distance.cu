@@ -10,8 +10,6 @@
 // Roofline: HBM.  The fp64 pipe does 3 (unweighted) or 4 (weighted) issue slots per element,
 // ~20 % of the memory time at D=128 on B200, so the kernel is bandwidth bound as long as
 // the TMA pipeline keeps >= ~45 KiB in flight per SM (see rowstream.cuh).
-#include <cstdlib>
-
 #include "rowstream.cuh"
 
 extern "C" int elfi_b200_colmoments_f64(elfi_b200_ctx* ctx, const double* S, int64_t ldS, int64_t B,
@@ -311,12 +309,11 @@ colmoments_flush_kernel(const double* __restrict__ S, const double* __restrict__
 // accumulators (two warps per scheduler leave the fp64 pipe half idle: long dependent chains of
 // K + 2 accumulators per lane), else 8.  Measured at 5e5 x 256: K = 2 0.232 -> 0.214 ms, K = 6
 // 0.297 -> 0.279 ms; 16 warps (128 registers, 2-slot ring) gives the 8-warp time back, and the
-// plain nested kernels do not gain from either.  ELFI_B200_FUSED_WARPS=8 restores 8 (KMAX <= 8).
+// plain nested kernels do not gain from either.
 template <int KMAX>
 static int fused_moments_warps(elfi_b200_ctx* ctx, int64_t Dp, int64_t K) {
-    int warps = 12;
-    if (const char* e = getenv("ELFI_B200_FUSED_WARPS")) warps = atoi(e);
-    if (KMAX > 8 || warps != 12) return RS_WARPS;
+    constexpr int warps = 12;
+    if (KMAX > 8) return RS_WARPS;
     const size_t aux = NestedMomentsConsumer<KMAX>::aux_bytes(Dp, K, warps);
     return rs_pick_stages(ctx->smem_optin, aux, warps) >= 3 ? warps : RS_WARPS;
 }

@@ -17,14 +17,13 @@
 // Variance uses the explicit inverse factor W = L^-1 instead of a triangular solve per query
 // chunk:  v_i = k** - || W k_i ||^2.  The product is a GEMM with a triangular K-range (row a
 // of W is zero beyond column a), i.e. n^2 m / 2 FMAs = 0.4 TFLOP at n = 2000, m = 1e5.
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace elfi {
 
 constexpr int GP_NB = 64;          // Cholesky panel width / base block of the inverse
 constexpr int GM_BM = 128, GM_BN = 128;
+constexpr int GM_SMALL_BELOW = 100;   // products with fewer large tiles take the 64 x 64 instance
 // k-slab width BK (16 or 32); smem rows are padded to BK + 4 doubles: the 16 lanes of a half warp
 // (grp 0..3 x tig 0..3) then read 16 distinct 8-byte banks
 constexpr int GM_STAGES = 3;       // cp.async ring: two slabs in flight while one is consumed
@@ -54,25 +53,27 @@ struct GemmArgs {
     int mode;   // 0 full; 1 lower tiles only (SYRK-style); 2 K limited to col0 + BN (B lower-tri)
     // mode 2 only: B is lower triangular with EXACT zeros above the diagonal and only its first
     // n_valid rows matter (rows >= n_valid belong to the identity padding and meet zero columns of
-    // A).  When tri_skip is set a warp skips the DMMA steps that would only multiply those zeros:
-    // k > c for all 8 columns c of a sub-tile, and whole sub-tiles of columns >= n_valid.
-    int tri_skip; int64_t n_valid;
+    // A).  A warp skips the DMMA steps that would only multiply those zeros: k > c for all 8
+    // columns c of a sub-tile, and whole sub-tiles of columns >= n_valid.
+    int64_t n_valid;
     // When set, C is not stored: the CTA of column tile bx writes, for each of its rows r,
     // rowsq[bx * ld_rowsq + r] = sum over the tile's columns of (A B^T)[r][c]^2 (alpha must be 1,
     // beta 0) -- the predictive variance needs |W k_i|^2, not W k_i.
     double* rowsq; int64_t ld_rowsq;
 };
 
-// C = alpha * A * B^T + beta * C on the fp64 tensor path.  CTA tile BM x BN x 16, WARPS_M x WARPS_N
+// C = alpha * A * B^T + beta * C on the fp64 tensor path.  CTA tile BM x BN x BK, WARPS_M x WARPS_N
 // warps, each a (BM / WARPS_M) x (BN / WARPS_N) tile of 8x8 DMMA tiles; 3-stage cp.async ring with
-// ONE block barrier per 16-wide slab (round 1: double buffering with two barriers, during which
+// ONE block barrier per BK-wide slab (round 1: double buffering with two barriers, during which
 // the tensor pipe idled: ncu showed `wait` / `math_pipe_throttle` stalls at 58 % of the DMMA
-// peak); batch = grid.z.  Two instances:
-//   128 x 128, 2 x 4 warps  -- the n^2 m / 2 prediction product and the large trailing updates;
-//    64 x  64, 2 x 2 warps  -- products with fewer than ~100 large tiles (the next-block-column
-//                              update of every Cholesky panel: 128 x 64 x 64 useful per CTA in a
-//                              128 x 128 tile; the levels of the recursive inverse: at most 64
-//                              large tiles on 148 SMs): four times the CTAs, three CTAs per SM.
+// peak); batch = grid.z.  Two tile shapes:
+//   128 x 128, 2 x 4 warps, BK 32  -- the n^2 m / 2 prediction product (the TRI instance) and the
+//                                     large trailing updates;
+//    64 x  64, 2 x 2 warps, BK 16  -- products with fewer than GM_SMALL_BELOW large tiles (the
+//                                     next-block-column update of every Cholesky panel: 128 x 64
+//                                     x 64 useful per CTA in a 128 x 128 tile; the levels of the
+//                                     recursive inverse: at most 64 large tiles on 148 SMs): four
+//                                     times the CTAs, three CTAs per SM.
 // (mma.m16n8k16.f64 is no alternative: ptxas lowers it to eight DMMA.8 on sm_100a,
 // profiles/r2_dmma_m16n8k16_sass.md.)
 template <int BM, int BN, int WARPS_M, int WARPS_N, int BK>
@@ -118,7 +119,7 @@ gemm_nt_dmma_kernel(GemmArgs g) {
     constexpr int CSTR = 8 * WARPS_N;
     int klast[TN];          // last k at which sub-tile j still meets a non-zero of B
     int klast_min = 0x7fffffff;
-    const bool tri = TRI && g.mode == 2;   // TRI instances are launched for tri_skip products only
+    const bool tri = TRI && g.mode == 2;   // TRI instances are launched for mode-2 products only
 #pragma unroll
     for (int j = 0; j < TN; ++j) {
         const int64_t c0 = col0 + j * CSTR + wn * 8;
@@ -270,25 +271,14 @@ static int launch_gemm_cfg(const GemmArgs& g, int64_t batch, cudaStream_t stream
 
 static int launch_gemm(const GemmArgs& g, int64_t batch, cudaStream_t stream) {
     if (g.M <= 0 || g.N <= 0 || batch <= 0) return ELFI_B200_OK;
-    static const int small_below = [] {
-        const char* v = getenv("ELFI_B200_GEMM_SMALL_BELOW");   // 0 = always the large tile
-        return v ? atoi(v) : 100;
-    }();
     int64_t tiles = ((g.M + GM_BM - 1) / GM_BM) * ((g.N + GM_BN - 1) / GM_BN) * batch;
     if (g.mode == 1) tiles = tiles / 2 + 1;
-    if (g.mode != 2 && tiles < small_below) return launch_gemm_cfg<64, 64, 2, 2, 16>(g, batch, stream);
+    if (g.mode != 2 && tiles < GM_SMALL_BELOW) return launch_gemm_cfg<64, 64, 2, 2, 16>(g, batch, stream);
     // 32-wide slabs halve the block barriers of the large tile (221 KB of shared memory, 230
-    // registers): the 1e5 x 2000 grid prediction 16.40 -> 15.96 ms.  ELFI_B200_GEMM_BK32=0: 16.
-    static const bool wide_slab = [] {
-        const char* v = getenv("ELFI_B200_GEMM_BK32");
-        return !(v != nullptr && v[0] == '0');
-    }();
-    if (g.mode == 2 && g.tri_skip) {   // the guarded k-steps exist in these two instances only
-        if (wide_slab) return launch_gemm_cfg<GM_BM, GM_BN, 2, 4, 32, true>(g, batch, stream);
-        return launch_gemm_cfg<GM_BM, GM_BN, 2, 4, 16, true>(g, batch, stream);
-    }
-    if (wide_slab) return launch_gemm_cfg<GM_BM, GM_BN, 2, 4, 32>(g, batch, stream);
-    return launch_gemm_cfg<GM_BM, GM_BN, 2, 4, 16>(g, batch, stream);
+    // registers): the 1e5 x 2000 grid prediction 16.40 -> 15.96 ms against 16-wide slabs.
+    if (g.mode == 2)   // the guarded k-steps exist in this instance only
+        return launch_gemm_cfg<GM_BM, GM_BN, 2, 4, 32, true>(g, batch, stream);
+    return launch_gemm_cfg<GM_BM, GM_BN, 2, 4, 32>(g, batch, stream);
 }
 
 // ---- K10: Gram / cross-covariance ----------------------------------------------------------
@@ -736,14 +726,12 @@ int elfi_b200_gp_fit_f64(elfi_b200_ctx* ctx, const double* X, int64_t ldX, const
     // caller's stream right away, the rest of the trailing matrix on the context's side stream,
     // where it overlaps with the next panel's latency-bound factorisation.  Ordering: the side
     // stream waits for the panel (ev_panel); the caller's stream waits for rest(p - 1) before it
-    // touches block column p + 1 again (ev_rest).  ELFI_B200_GP_LOOKAHEAD=0: one stream.
+    // touches block column p + 1 again (ev_rest).  One stream (panel + one SYRK of the whole
+    // trailing matrix) is slower: 2.54 against 2.48 ms per fit at n = 2000, 8.47 against 8.07 ms at
+    // n = 4000 (B200, 1000 W power limit; DESIGN.md section 6).
     double* T = static_cast<double*>(ctx_scratch(ctx, size_t(n_pad) * n_pad * 8 + 256));
     if (!T) return ELFI_B200_ERR_NOMEM;
     double* Dblocks = T;     // (n_pad / 64) factored diagonal blocks, copied into L after the loop
-    static const bool lookahead = [] {
-        const char* v = getenv("ELFI_B200_GP_LOOKAHEAD");
-        return !(v != nullptr && v[0] == '0');
-    }();
     cudaStream_t side = ctx->copy_stream[0];
     cudaEvent_t ev_panel = ctx->copy_event[0], ev_rest = ctx->copy_event[1];
     bool rest_pending = false;
@@ -767,11 +755,6 @@ int elfi_b200_gp_fit_f64(elfi_b200_ctx* ctx, const double* X, int64_t ldX, const
         }
         potrf_diag_panel_kernel<<<unsigned((below + 127) / 128), 128, 0, stream>>>(
             L, n_pad, k, n_pad, info, Dblocks + (k / GP_NB) * GP_NB * GP_NB);
-        if (!lookahead) {
-            int rc = syrk(k, k + GP_NB, below, below, 1, stream);
-            if (rc) return rc;
-            continue;
-        }
         ELFI_CUDA_OK(cudaEventRecord(ev_panel, stream));
         if (rest_pending) { ELFI_CUDA_OK(cudaStreamWaitEvent(stream, ev_rest, 0)); rest_pending = false; }
         int rc = syrk(k, k + GP_NB, below, GP_NB, 0, stream);          // next block column
@@ -877,12 +860,8 @@ int elfi_b200_gp_predict_f64(elfi_b200_ctx* ctx, const double* Xq, int64_t ldq, 
     // its GEMM plus the K* / epilogue kernels' launch gaps, so chunks are as large as gridDim.y of
     // the K* kernel allows (32768 rows = 0.5 GB of scratch at n_pad = 2048, nothing on a 180 GB
     // part) and equal in size (a short last chunk would be 1-2 ragged waves).  Round 2 ran 8192-row
-    // chunks; ELFI_B200_GP_PREDICT_CHUNK restores any other size.
-    static const int64_t mc_max = [] {
-        const char* v = getenv("ELFI_B200_GP_PREDICT_CHUNK");
-        const long c = v ? atol(v) : 32768;
-        return int64_t(c < 128 ? 128 : (c > 65408 ? 65408 : c));
-    }();
+    // chunks (profiles/r2_gp_predict_tri_skip.md).
+    constexpr int64_t mc_max = 32768;
     const int64_t nchunks = (m + mc_max - 1) / mc_max;
     const int64_t mc = ((m + nchunks - 1) / nchunks + 127) / 128 * 128;
     // scratch: Ks (mc x n_pad), then the per-column-tile sums of squares (ntiles x mc)
@@ -902,14 +881,9 @@ int elfi_b200_gp_predict_f64(elfi_b200_ctx* ctx, const double* Xq, int64_t ldq, 
         g.B = W; g.ldb = n_pad;
         g.C = nullptr; g.ldc = n_pad;          // V = K* W^T is consumed in the epilogue
         g.rowsq = rowsq; g.ld_rowsq = mc;
-        g.M = rows; g.N = n_pad; g.K = n_pad; g.alpha = 1.0; g.beta = 0.0; g.mode = 2;
-        static const bool tri_skip = [] {
-            const char* v = getenv("ELFI_B200_GEMM_TRI_SKIP");
-            return !(v != nullptr && v[0] == '0');
-        }();
-        g.tri_skip = tri_skip ? 1 : 0;
+        // k >= n: zero columns of K*, identity rows of W
+        g.M = rows; g.N = n_pad; g.K = (n + 3) & ~int64_t(3); g.alpha = 1.0; g.beta = 0.0; g.mode = 2;
         g.n_valid = n;
-        if (tri_skip) g.K = (n + 3) & ~int64_t(3);   // k >= n: zero columns of K*, identity rows of W
         int rc = launch_gemm(g, 1, stream);
         if (rc) return rc;
         predict_rows_sq_kernel<<<unsigned((rows + 7) / 8), 256, 0, stream>>>(

@@ -10,8 +10,6 @@
 // (<= 2e6 pairs = 24 MB) are L2 resident, so the sort is latency/issue bound, not HBM bound;
 // passes whose digit is constant over all keys (typical for the high exponent bits of
 // distances) degenerate to a copy.
-#include <cstdlib>
-
 #include "eqweight.h"
 #include "pairwise.cuh"
 
@@ -975,7 +973,7 @@ int elfi_b200_rowsort_f64(elfi_b200_ctx* ctx, const double* X, int64_t ldX, int6
     ELFI_CUDA_OK(cudaSetDevice(ctx->device));
     int npow2 = 2;
     while (npow2 < n) npow2 <<= 1;
-    if (npow2 <= 512 && getenv("ELFI_B200_ROWSORT_SMEM") == nullptr) {
+    if (npow2 <= 512) {
         const int kpl = npow2 <= 32 ? 1 : npow2 / 32;
         switch (kpl) {
             case 1: launch_rowsort_regs<1>(X, ldX, B, int(n), out, ld_out, ctx->sm_count, stream); break;

@@ -12,8 +12,6 @@
 //                                 rejection of draws outside the prior support)
 // The random numbers are a pure function of (seed, stream, row, index): the simulator can be
 // replayed (e.g. to materialise X for a test) and any sharding of rows gives the same particles.
-#include <cstdlib>
-
 #include "gnkmath.cuh"
 #include "leafsum.cuh"
 #include "pairwise.cuh"
@@ -484,7 +482,7 @@ int elfi_b200_sim_ma2_f64(elfi_b200_ctx* ctx, const double* t1, const double* t2
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
     ELFI_CUDA_OK(cudaSetDevice(ctx->device));
     const unsigned blocks = unsigned((B + 127) / 128);
-    const bool leaf = n_obs - 1 <= LEAF_MAX_TERMS && getenv("ELFI_B200_SIM_MA2_TREE") == nullptr;
+    const bool leaf = n_obs - 1 <= LEAF_MAX_TERMS;
 #define ELFI_SIM_MA2(WX, SM, LF) \
     sim_ma2_kernel<WX, SM, LF><<<blocks, 128, 0, stream>>>(t1, t2, B, int(n_obs), seed, offset, X, ldX, S, ldS)
     if (X && S) { if (leaf) ELFI_SIM_MA2(true, true, true); else ELFI_SIM_MA2(true, true, false); }
@@ -597,7 +595,7 @@ int elfi_b200_sim_gauss_f64(elfi_b200_ctx* ctx, const double* mu, const double* 
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
     ELFI_CUDA_OK(cudaSetDevice(ctx->device));
     const unsigned blocks = unsigned((B + 127) / 128);
-    const bool leaf = n_obs <= LEAF_MAX_TERMS && getenv("ELFI_B200_SIM_GAUSS_TREE") == nullptr;
+    const bool leaf = n_obs <= LEAF_MAX_TERMS;
 #define ELFI_SIM_GAUSS(WY, LF) \
     sim_gauss_kernel<WY, LF><<<blocks, 128, 0, stream>>>(mu, sigma, B, int(n_obs), seed, offset, Y, ldY, S, ldS)
     if (Y) { if (leaf) ELFI_SIM_GAUSS(true, true); else ELFI_SIM_GAUSS(true, false); }

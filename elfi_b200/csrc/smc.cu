@@ -12,8 +12,6 @@
 // 64-bit conversions, which run at quarter rate) and a degree-6 minimax polynomial: relative
 // error < 2e-9 per term, far inside the 1e-5 relative tolerance on the weights.  Accumulation
 // is fp64.
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace elfi {
@@ -162,7 +160,7 @@ __device__ __forceinline__ double exp2_neg(double nt) {
     return (nt <= 1020.0) ? r : 0.0;
 }
 
-// Mixed-precision variant of exp2_neg (opt-in, ELFI_B200_GM_MODE=mixed): the range reduction
+// Mixed-precision variant of exp2_neg (elfi_b200_gm_logpdf_mixed_f64): the range reduction
 // stays in fp64 (the integer / fraction split of nt needs it), but 2^f for f in [-.5, .5] comes
 // from the special-function unit in fp32 (ex2.approx: 2 ulp, ~1.7e-7 relative) and is widened
 // back to fp64 with integer operations while the exponent k is added -- no polynomial: the
@@ -350,7 +348,7 @@ int elfi_b200_weighted_stats_f64(elfi_b200_ctx* ctx, const double* x, int64_t ld
 static int gm_logpdf_impl(elfi_b200_ctx* ctx, const double* x, int64_t ldx, int64_t N,
                           const double* means, int64_t ldm, const double* w, int64_t M, int64_t p,
                           const double* Linv_host, double logdet, double* logq, void* stream_,
-                          bool mixed_entry) {
+                          bool mixed) {
     using namespace elfi;
     ELFI_REQUIRE(ctx && x && means && Linv_host && logq, "gm_logpdf: NULL argument");
     ELFI_REQUIRE(N >= 0 && M >= 1 && p >= 1 && p <= WS_MAXP && ldx >= p && ldm >= p,
@@ -371,10 +369,6 @@ static int gm_logpdf_impl(elfi_b200_ctx* ctx, const double* x, int64_t ldx, int6
         chunk_len = ((M / 64 + 511) / 512) * 512;
         if (chunk_len < 2048) chunk_len = 2048;
         if (chunk_len > 16384) chunk_len = 16384;
-        if (const char* e = getenv("ELFI_B200_GM_CHUNK")) {
-            const long v = atol(e);
-            if (v >= 512) chunk_len = (int64_t(v) / 512) * 512;
-        }
         chunks = (M + chunk_len - 1) / chunk_len;
         ELFI_REQUIRE(chunks <= 65535, "gm_logpdf: too many component chunks (%lld)", (long long)chunks);
     }
@@ -398,12 +392,6 @@ static int gm_logpdf_impl(elfi_b200_ctx* ctx, const double* x, int64_t ldx, int6
     const double lognorm = -0.5 * (double(p) * 1.8378770664093453 + logdet);  // log(2 pi)
     if (p <= 4) {
         dim3 grid(static_cast<unsigned>(xblocks), static_cast<unsigned>(chunks));
-        // ELFI_B200_GM_MODE = fp64 | mixed overrides the choice of the entry point (measurements)
-        static const int forced = [] {
-            const char* v = getenv("ELFI_B200_GM_MODE");
-            return v == nullptr ? 0 : (v[0] == 'm' ? 2 : (v[0] == 'f' ? 1 : 0));
-        }();
-        const bool mixed = forced == 2 || (forced == 0 && mixed_entry);
         if (mixed) {
             switch (p) {
                 case 1: gm_pdf_kernel<1, R, true><<<grid, 128, 0, stream>>>(xw, N, mw, M, chunk_len, partial); break;

@@ -6,9 +6,10 @@
 // 8 strided accumulators r[0..7] combined as ((r0+r1)+(r2+r3))+((r4+r5)+(r6+r7)) plus a
 // sequential tail; longer rows are split recursively at n/2 rounded down to a multiple of 8.
 // Every left part is a multiple of 8 long, so every leaf starts at an index that is a multiple
-// of 8 and only the last leaf has a tail.  PairwiseStream below consumes a row's terms strictly
-// in order and reproduces that tree bit for bit, with the accumulators indexed by compile-time
-// constants (the term index modulo 8 is fixed by the column position and the lag).
+// of 8 and only the last leaf has a tail.  The row-stream consumers below reproduce that tree bit
+// for bit with the accumulators of leafsum.cuh / treesum.cuh, indexed by compile-time constants
+// (the term index modulo 8 is fixed by the column position and the lag); the generic fallback
+// feeds the same tree through PairwiseStream (pairwise.cuh).
 //
 // Traffic: n*8 bytes read per row (variance re-reads the tile from L2), 8 bytes written per
 // statistic.  Roofline: HBM.
@@ -17,39 +18,9 @@
 #include "rowstream.cuh"
 #include "treesum.cuh"
 
-#include <cstdlib>
-
 namespace elfi {
 
-// Collects terms into aligned groups of 8 and forwards them to a PairwiseStream.
 constexpr int RS_PW_DEPTH = 6;   // rows of up to 7688 terms on the row-stream path (max_terms())
-
-struct TermGrouper {
-    PairwiseStream<RS_PW_DEPTH> pw;
-    double buf[8];
-    int j0;
-    int fill;
-    __device__ __forceinline__ void begin(int m) {
-        pw.begin(m);
-        j0 = 0;
-        fill = 0;
-    }
-    template <int K>
-    __device__ __forceinline__ void push(double v) {  // K = term index modulo 8 (compile time)
-        buf[K] = v;
-        if (K == 7) {
-            pw.feed8(j0, buf, 8);
-            j0 += 8;
-            fill = 0;
-        } else {
-            fill = K + 1;
-        }
-    }
-    __device__ __forceinline__ double finish() {
-        if (fill > 0) pw.feed8(j0, buf, fill);
-        return __dadd_rn(0.0, pw.finish());   // np.add.reduce starts from the identity 0.0
-    }
-};
 
 struct SummaryParams {
     double* out;      // out[row * ld_out + col0 (+1)]
@@ -68,106 +39,11 @@ __device__ __forceinline__ void load_box_row(const uint8_t* box_row, int sw, dou
     }
 }
 
-// Autocovariance at one or two compile-time lags in a single pass over the rows:
-// C_lag = mean_j( x[j+lag] * x[j] ),  j = 0 .. n-lag-1   (ma2.py:57: np.mean(x[:,lag:]*x[:,:-lag])).
-template <int LAG_A, int LAG_B>
-struct AutocovConsumer {
-    typedef SummaryParams Params;
-    static constexpr int PASSES = 1;
-    static constexpr int HMAX = (LAG_A > LAG_B ? LAG_A : LAG_B);
-    const Params& p;
-    TermGrouper ga, gb;
-    double hist[HMAX > 0 ? HMAX : 1];  // last HMAX elements of the previous column group
-
-    static __device__ void setup_shared(uint8_t*, const Params&, int) {}
-    __device__ AutocovConsumer(const Params& p_, const uint8_t*, int, int) : p(p_) {}
-    __device__ __forceinline__ void begin_row() {
-        ga.begin(p.n - LAG_A);
-        if (LAG_B >= 0) gb.begin(p.n - LAG_B);
-    }
-    template <int LAG, int C>
-    __device__ __forceinline__ void term(TermGrouper& g, int t, const double* cur) {
-        // element index t = cg*16 + C; product index j = t - LAG
-        if (t >= LAG && t < p.n) {
-            const double prev = (C >= LAG) ? cur[C >= LAG ? C - LAG : 0]
-                                           : hist[C >= LAG ? 0 : HMAX - LAG + C];
-            g.template push<((C - LAG) % 8 + 8) % 8>(__dmul_rn(cur[C], prev));
-        }
-    }
-    template <int C>
-    __device__ __forceinline__ void step(int t0, const double* cur) {
-        term<LAG_A, C>(ga, t0 + C, cur);
-        if (LAG_B >= 0) term<(LAG_B >= 0 ? LAG_B : 0), C>(gb, t0 + C, cur);
-        if constexpr (C + 1 < 16) step<C + 1>(t0, cur);
-    }
-    __device__ __forceinline__ void consume(int, int cg, const uint8_t* box_row, int sw) {
-        double cur[16];
-        load_box_row(box_row, sw, cur);
-        step<0>(cg * RS_BOX_COLS, cur);
-#pragma unroll
-        for (int h = 0; h < HMAX; ++h) hist[h] = cur[16 - HMAX + h];
-    }
-    __device__ __forceinline__ void end_row(int64_t row, int64_t B, int) {
-        const double sa = ga.finish();
-        double sb = 0.0;
-        if (LAG_B >= 0) sb = gb.finish();
-        if (row < B) {
-            p.out[row * p.ld_out + p.col_a] = sa / double(p.n - LAG_A);
-            if (LAG_B >= 0) p.out[row * p.ld_out + p.col_b] = sb / double(p.n - LAG_B);
-        }
-    }
-};
-
-// np.mean / np.var along axis 1 (gauss.py:156, 173).  Sweep 0 accumulates the pairwise sum
-// of x; sweep 1 (same boxes, L2 hits) the pairwise sum of (x - mean)^2  (numpy _var).
-struct MeanVarConsumer {
-    typedef SummaryParams Params;
-    static constexpr int PASSES = 2;
-    const Params& p;
-    TermGrouper g;
-    double mean;
-
-    static __device__ void setup_shared(uint8_t*, const Params&, int) {}
-    __device__ MeanVarConsumer(const Params& p_, const uint8_t*, int, int) : p(p_), mean(0.0) {}
-    __device__ __forceinline__ void begin_row() { g.begin(p.n); }
-    template <int C>
-    __device__ __forceinline__ void step(int pass, int t0, const double* cur) {
-        if (t0 + C < p.n) {
-            if (pass == 0) {
-                g.template push<C % 8>(cur[C]);
-            } else {
-                const double c = __dsub_rn(cur[C], mean);
-                g.template push<C % 8>(__dmul_rn(c, c));
-            }
-        }
-        if constexpr (C + 1 < 16) step<C + 1>(pass, t0, cur);
-    }
-    __device__ __forceinline__ void consume(int pass, int cg, const uint8_t* box_row, int sw) {
-        double cur[16];
-        load_box_row(box_row, sw, cur);
-        if (pass == 1 && cg == 0) {
-            mean = g.finish() / double(p.n);
-            g.begin(p.n);
-        }
-        step<0>(pass, cg * RS_BOX_COLS, cur);
-    }
-    __device__ __forceinline__ void end_row(int64_t row, int64_t B, int) {
-        const double var = g.finish() / double(p.n);
-        if (row < B) {
-            if (p.col_a >= 0) p.out[row * p.ld_out + p.col_a] = mean;
-            if (p.col_b >= 0) p.out[row * p.ld_out + p.col_b] = var;
-        }
-    }
-};
-
-// Term-wise variants: the per-lane state is one of the accumulators of leafsum.cuh / treesum.cuh
+// Term-wise consumers: the per-lane state is one of the accumulators of leafsum.cuh / treesum.cuh
 // and the box logic is AutocovBoxes / MeanVarBoxes, which also compile for the host.
 //   Sum = LeafSum   every reduced run has <= 128 terms, so NumPy's tree is one leaf and the state
-//                   is 8 accumulators per sum: same results as the consumers above at a fraction
-//                   of the integer bookkeeping (profiles/r1_summ_instruction_mix.md).  Default.
-//   Sum = TreeSum   longer rows, same front end; default for rows of more than 128 terms since its
-//                   device timing (ELFI_B200_SUMM_TERMWISE=0 falls back to the TermGrouper
-//                   consumers).
+//                   is 8 accumulators per sum (profiles/r1_summ_instruction_mix.md).
+//   Sum = TreeSum   rows of 129..7688 terms, same front end.
 template <class Sum, int LAG_A, int LAG_B>
 struct AutocovBoxConsumer {
     typedef SummaryParams Params;
@@ -345,11 +221,7 @@ static size_t rg_smem_bytes(int warps, int ns, int64_t n) {
 }
 
 static bool rowgroup_ok(elfi_b200_ctx* ctx, const double* X, int64_t ld, int64_t n) {
-    static const bool off = [] {
-        const char* v = std::getenv("ELFI_B200_MEANVAR_ROWGROUP");
-        return v != nullptr && v[0] == '0';
-    }();
-    if (off || ld != n || n > 64 || (n & 3) != 2 || (reinterpret_cast<uintptr_t>(X) & 15)) return false;
+    if (ld != n || n > 64 || (n & 3) != 2 || (reinterpret_cast<uintptr_t>(X) & 15)) return false;
     return rg_smem_bytes(6, 2, n) + 1024 <= ctx->smem_optin;
 }
 
@@ -380,20 +252,12 @@ static int rowgroup_launch(elfi_b200_ctx* ctx, const double* X, int64_t B, int64
 
 typedef TreeSum<RS_PW_DEPTH> RowTreeSum;
 
-// Rows of 129..7688 terms: the term-wise TreeSum front end is the default since it was timed on
-// the device (autocov(1,2) 4e5 x 256: 0.152 ms = 0.83 of the HBM peak against 0.225 ms = 0.56 for
-// the TermGrouper consumers; mean/var 0.183 against 0.350 ms; profiles/r2_kernels.md).
-// ELFI_B200_SUMM_TERMWISE=0 selects the round-1 consumers.
-static bool summaries_termwise() {
-    static const bool on = [] {
-        const char* v = std::getenv("ELFI_B200_SUMM_TERMWISE");
-        return !(v != nullptr && v[0] == '0');
-    }();
-    return on;
-}
+// Rows of 129..7688 terms take the term-wise TreeSum front end (autocov(1,2) 4e5 x 256: 0.152 ms =
+// 0.83 of the HBM peak against 0.225 ms = 0.56 for the round-1 group-of-8 consumers; mean/var
+// 0.183 against 0.350 ms; profiles/r2_kernels.md).
 
 // Generic fallback (any lag, any alignment): one thread per row straight from global memory,
-// same PairwiseStream so results are identical.  mode 0 = autocov(lag), 1 = mean+var.
+// same tree through PairwiseStream so results are identical.  mode 0 = autocov(lag), 1 = mean+var.
 __global__ void __launch_bounds__(128)
 summary_direct_kernel(const double* __restrict__ X, int64_t ld, int64_t B, int n, int lag,
                       int mode, SummaryParams p) {
@@ -438,10 +302,7 @@ static int autocov_launch(elfi_b200_ctx* ctx, const double* X, int64_t ld, int64
                           const SummaryParams& p, cudaStream_t stream) {
     if (n - LA <= LEAF_MAX_TERMS)   // LA is the smaller lag: the longer run
         return rowstream_launch<AutocovBoxConsumer<LeafSum, LA, LB>>(ctx, X, ld, B, n, 0, p, stream);
-    if (summaries_termwise())
-        return rowstream_launch<AutocovBoxConsumer<RowTreeSum, LA, LB>>(ctx, X, ld, B, n, 0, p,
-                                                                        stream);
-    return rowstream_launch<AutocovConsumer<LA, LB>>(ctx, X, ld, B, n, 0, p, stream);
+    return rowstream_launch<AutocovBoxConsumer<RowTreeSum, LA, LB>>(ctx, X, ld, B, n, 0, p, stream);
 }
 
 }  // namespace elfi
@@ -531,18 +392,13 @@ int elfi_b200_summary_meanvar_f64(elfi_b200_ctx* ctx, const double* X, int64_t l
         return rowgroup_launch<4>(ctx, X, B, n, p, stream);
     }
     if (rowstream_ok(ctx, X, ldX, n)) {
-        static const bool two_sweeps = std::getenv("ELFI_B200_MEANVAR_TWO_SWEEPS") != nullptr;
-        if (!two_sweeps) {
-            if (n <= 16) return rowstream_launch<MeanVarRegsConsumer<1>>(ctx, X, ldX, B, n, 0, p, stream);
-            if (n <= 32) return rowstream_launch<MeanVarRegsConsumer<2>>(ctx, X, ldX, B, n, 0, p, stream);
-            if (n <= 48) return rowstream_launch<MeanVarRegsConsumer<3>>(ctx, X, ldX, B, n, 0, p, stream);
-            if (n <= 64) return rowstream_launch<MeanVarRegsConsumer<4>>(ctx, X, ldX, B, n, 0, p, stream);
-        }
+        if (n <= 16) return rowstream_launch<MeanVarRegsConsumer<1>>(ctx, X, ldX, B, n, 0, p, stream);
+        if (n <= 32) return rowstream_launch<MeanVarRegsConsumer<2>>(ctx, X, ldX, B, n, 0, p, stream);
+        if (n <= 48) return rowstream_launch<MeanVarRegsConsumer<3>>(ctx, X, ldX, B, n, 0, p, stream);
+        if (n <= 64) return rowstream_launch<MeanVarRegsConsumer<4>>(ctx, X, ldX, B, n, 0, p, stream);
         if (n <= LEAF_MAX_TERMS)
             return rowstream_launch<MeanVarBoxConsumer<LeafSum>>(ctx, X, ldX, B, n, 0, p, stream);
-        if (summaries_termwise())
-            return rowstream_launch<MeanVarBoxConsumer<RowTreeSum>>(ctx, X, ldX, B, n, 0, p, stream);
-        return rowstream_launch<MeanVarConsumer>(ctx, X, ldX, B, n, 0, p, stream);
+        return rowstream_launch<MeanVarBoxConsumer<RowTreeSum>>(ctx, X, ldX, B, n, 0, p, stream);
     }
     summary_direct_kernel<<<unsigned((B + 127) / 128), 128, 0, stream>>>(X, ldX, B, int(n), 0, 1, p);
     ELFI_CUDA_OK(cudaGetLastError());

@@ -4,8 +4,7 @@
 // (leafsum.cuh): terms arrive one at a time with their index modulo 8 known at compile time, so
 // a column group whose 16 terms fall inside the whole-groups range of the current leaf takes the
 // branch-free path, and the recursion stack is only touched once per <= 128-term leaf.  The
-// row-stream summary kernels can use it for rows of 129..7688 terms instead of the
-// group-of-8 TermGrouper front end (opt-in, see summaries.cu).
+// row-stream summary kernels use it for rows of 129..7688 terms (see summaries.cu).
 //
 // NumPy (DOUBLE_pairwise_sum): n <= 128 is a leaf (8 strided accumulators + sequential tail);
 // longer runs split at n/2 rounded down to a multiple of 8, left part first.  Every left part is

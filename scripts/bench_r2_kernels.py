@@ -112,7 +112,7 @@ for N in (125_000, 1_000_000):
              tflops_equiv=N * M * 16 / (ms * 1e-3) / 1e12)
     out.append(e)
     print(json.dumps(e), flush=True)
-    if N == 125_000:      # kept for an accuracy comparison between ELFI_B200_GM_MODE variants
+    if N == 125_000:
         np.save(os.path.join(ROOT, 'gpurun_out', 'gm_logq_{}.npy'.format(TAG)),
                 ops.gm_logpdf(xs, means, cov, w, validate=False).cpu().numpy())
 

@@ -1,23 +1,19 @@
 #!/usr/bin/env python
-"""GP grid prediction (m = 1e5, n = 2000) with and without the triangular DMMA skip
-(ELFI_B200_GEMM_TRI_SKIP=0 multiplies the zeros above W's diagonal and the padded columns as
-before).  One process per variant (the switch is static); the parent compares the two variants'
-outputs (they must agree to the last bit: only products with exact zeros are skipped) and both
-against a float64 NumPy/SciPy evaluation on a sub-grid."""
+"""GP grid prediction (m = 1e5 points, n = 2000, 2048 and 700 training points) and the n = 2000
+fit, timed with CUDA events; the predictions are checked against a float64 NumPy evaluation on a
+sub-grid."""
 import ctypes
 import json
 import os
-import subprocess
 import sys
 
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-OUT = os.path.join(ROOT, 'gpurun_out')
 
 
-def child(tag):
+def main():
     import torch
     from elfi_b200 import _lib, device as dev
     from elfi_b200.bo import GPyRegression
@@ -44,7 +40,7 @@ def child(tag):
                 b.record()
                 torch.cuda.synchronize()
                 ft.append(a.elapsed_time(b) / 3)
-            print(json.dumps(dict(name='gp_fit_n2000', variant=tag, ms_median=float(np.median(ft)),
+            print(json.dumps(dict(name='gp_fit_n2000', ms_median=float(np.median(ft)),
                                   ms_min=float(min(ft)))), flush=True)
         g1, g2 = np.meshgrid(np.linspace(-2, 2, 400), np.linspace(-1, 1, 250))
         grid_h = np.column_stack([g1.ravel(), g2.ravel()])
@@ -65,7 +61,6 @@ def child(tag):
         m = grid.shape[0]
         flops = (m * n * n / 2 + m * n) * 2.0
         mean, var = out[0].cpu().numpy(), out[1].cpu().numpy()
-        np.save(os.path.join(OUT, 'gp_predict_{}_n{}.npy'.format(tag, n)), np.stack([mean, var]))
         # float64 host evaluation of 500 grid points with the GP's own hyper-parameters
         h = gp.hyperparameters
         sub = np.linspace(0, m - 1, 500).astype(int)
@@ -78,9 +73,7 @@ def child(tag):
         sol = np.linalg.solve(Ky, np.column_stack([ye, Ks.T]))
         mean_h = Ks @ sol[:, 0]
         var_h = h['kernel_var'] + h['bias_var'] - np.einsum('ij,ji->i', Ks, sol[:, 1:])
-        res.append(dict(name='gp_predict_lcbsc_m1e5_n{}'.format(n), variant=tag,
-                        env={k: v for k, v in os.environ.items() if k.startswith('ELFI_B200_G')},
-                        ms_median=ms,
+        res.append(dict(name='gp_predict_lcbsc_m1e5_n{}'.format(n), ms_median=ms,
                         ms_min=float(min(ts)), TFLOPs=flops / ms / 1e9,
                         frac_dmma_peak=flops / ms / 1e9 / dmma, dmma_peak_tflops=dmma,
                         max_rel_err_mean=float(np.max(np.abs(mean[sub] - mean_h) /
@@ -90,22 +83,4 @@ def child(tag):
 
 
 if __name__ == '__main__':
-    if len(sys.argv) > 2 and sys.argv[1] == '--child':
-        child(sys.argv[2])
-    else:
-        os.makedirs(OUT, exist_ok=True)
-        # tag -> environment of the variant; the first one is the default configuration
-        variants = {'1': {}, '0': {'ELFI_B200_GEMM_TRI_SKIP': '0'}}
-        if '--chunks' in sys.argv:
-            variants = {'1': {}, '0': {'ELFI_B200_GP_PREDICT_CHUNK': '8192'}}
-        for tag, extra in variants.items():
-            env = dict(os.environ, **extra)
-            subprocess.check_call([sys.executable, os.path.abspath(__file__), '--child', tag], env=env)
-        for n in (2000, 2048, 700):
-            a = np.load(os.path.join(OUT, 'gp_predict_1_n{}.npy'.format(n)))
-            b = np.load(os.path.join(OUT, 'gp_predict_0_n{}.npy'.format(n)))
-            print(json.dumps(dict(name='variant_vs_default_n{}'.format(n), variants=variants,
-                                  identical=bool(np.array_equal(a, b)),
-                                  max_abs_diff=float(np.max(np.abs(a - b))))), flush=True)
-            os.remove(os.path.join(OUT, 'gp_predict_1_n{}.npy'.format(n)))
-            os.remove(os.path.join(OUT, 'gp_predict_0_n{}.npy'.format(n)))
+    main()

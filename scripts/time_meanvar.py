@@ -1,17 +1,16 @@
 #!/usr/bin/env python
-"""mean/var timings for contiguous rows: the 1-D bulk row-group kernel (n = 2 mod 4) against the
-2-D tensor-map row-stream path (ELFI_B200_MEANVAR_ROWGROUP=0).  The switch is read once per
-process, so the script re-runs itself per variant.  --once: a single launch (for ncu)."""
+"""mean/var timings for contiguous rows (n = 2 mod 4 takes the 1-D bulk row-group kernel, the
+other widths the 2-D tensor-map row-stream path), checked bit for bit against NumPy.
+--once: a single launch (for ncu)."""
 import json
 import os
-import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
 
-def child(once):
+def main(once):
     import numpy as np
     import torch
     from elfi_b200 import ops
@@ -44,18 +43,12 @@ def child(once):
         got = ops.meanvar(y[:4096].contiguous()).cpu().numpy()
         exact = bool(np.array_equal(got[:, 0], ref.mean(axis=1)) and
                      np.array_equal(got[:, 1], ref.var(axis=1)))
-        print(json.dumps(dict(name='meanvar_{}x{}'.format(B, n),
-                              rowgroup=os.environ.get('ELFI_B200_MEANVAR_ROWGROUP', '1'),
-                              ms_median=ms, ms_min=float(min(ts)), GBps=nbytes / ms / 1e6,
+        print(json.dumps(dict(name='meanvar_{}x{}'.format(B, n), ms_median=ms,
+                              ms_min=float(min(ts)), GBps=nbytes / ms / 1e6,
                               frac_hbm_measured=nbytes / ms / 1e6 / hbm, bit_exact=exact)),
               flush=True)
         del y
 
 
 if __name__ == '__main__':
-    if '--child' in sys.argv or '--once' in sys.argv:
-        child('--once' in sys.argv)
-    else:
-        for flag in ('1', '0'):
-            env = dict(os.environ, ELFI_B200_MEANVAR_ROWGROUP=flag)
-            subprocess.check_call([sys.executable, os.path.abspath(__file__), '--child'], env=env)
+    main('--once' in sys.argv)

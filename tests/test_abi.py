@@ -57,3 +57,15 @@ def test_product_never_imports_oracle():
                 if re.search(r'^\s*(import|from)\s+(elfi_oracle|oracle|ref_shim)\b', src, re.M):
                     bad.append(os.path.join(dirpath, f))
     assert not bad, bad
+
+
+def test_library_reads_no_environment():
+    """What the CUDA library computes depends on its arguments only, never on environment
+    variables of the process that loads it."""
+    bad = []
+    for top in (os.path.join(ROOT, 'elfi_b200', 'csrc'), os.path.join(ROOT, 'include')):
+        for dirpath, _, files in os.walk(top):
+            for f in files:
+                if 'getenv' in open(os.path.join(dirpath, f), errors='replace').read():
+                    bad.append(os.path.join(dirpath, f))
+    assert not bad, bad
