@@ -95,6 +95,8 @@ SIGNATURES = {
                                    c_i64, c_i64, c_i64, c_dbl, c_dbl, c_dbl, c_ptr, c_ptr],
     'elfi_b200_lcbsc_f64': [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_i64, c_dbl, c_ptr, c_ptr,
                             c_ptr],
+    'elfi_b200_synlik_f64': [c_ptr, ctypes.c_int32, c_ptr, c_i64, c_i64, c_i64, c_i64, c_i64, c_ptr,
+                             c_ptr, c_ptr, c_i64, c_ptr, c_ptr],
 }
 _SPECIAL_RESTYPE = {'elfi_b200_last_error': ctypes.c_char_p, 'elfi_b200_gp_padded_size': c_i64}
 _NO_STATUS = {'elfi_b200_version', 'elfi_b200_last_error', 'elfi_b200_ctx_sm_count',

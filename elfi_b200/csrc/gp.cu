@@ -18,6 +18,7 @@
 // chunk:  v_i = k** - || W k_i ||^2.  The product is a GEMM with a triangular K-range (row a
 // of W is zero beyond column a), i.e. n^2 m / 2 FMAs = 0.4 TFLOP at n = 2000, m = 1e5.
 #include "common.cuh"
+#include "dmma.cuh"
 
 namespace elfi {
 
@@ -36,12 +37,6 @@ __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc, boo
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-
-__device__ __forceinline__ void dmma_m8n8k4(double& c0, double& c1, double a, double b) {
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-                 : "+d"(c0), "+d"(c1)
-                 : "d"(a), "d"(b));
-}
 
 struct GemmArgs {
     const double* A; int64_t lda; int64_t strideA;   // (M, K) row-major

@@ -693,6 +693,51 @@ def kliep_fit(x, y, weights_x=None, weights_y=None, sigma=1.0, n_basis=100, epsi
     return alpha, float(res[0]), int(res[1])
 
 
+SYNLIK_ESTIMATORS = {'gaussian': 0, 'ghurye_olkin': 1}
+
+
+def synlik(S, obs, n, *, group_stride=None, estimator='gaussian', whitening=None, gammas=None):
+    """Gaussian synthetic log-likelihoods of groups of n simulated summary rows
+    (elfi/methods/bsl/pdf_methods.py:77-176) in one call of elfi_b200_synlik_f64.
+
+    S : (rows, d) array, group g = rows g * group_stride .. g * group_stride + n - 1 (group_stride
+        defaults to n; a row-strided view is read in place), or (P, n_rows, d) with group_stride
+        n_rows.
+    estimator : 'gaussian' or 'ghurye_olkin' (the unbiased estimator; no whitening / gammas).
+    whitening : (d, d) matrix Wh or None.
+    gammas : None (no shrinkage) or the L Warton parameters gamma = 1 - penalty (host values).
+
+    Returns a (P, L) device tensor; -inf for a group with non-finite values or a singular
+    covariance."""
+    if estimator not in SYNLIK_ESTIMATORS:
+        raise ValueError('unknown synthetic likelihood estimator {!r}'.format(estimator))
+    if dev.is_device_array(S) and S.dim() == 3 or not dev.is_device_array(S) and np.ndim(S) == 3:
+        S = dev.to_device(S)
+        if group_stride is None:
+            group_stride = S.shape[1]
+        S = S.reshape(-1, S.shape[2])
+    S = _matrix(S)
+    rows, d = S.shape
+    n = int(n)
+    gs = n if group_stride is None else int(group_stride)
+    P = (rows - n) // gs + 1 if rows >= n and gs > 0 else 0
+    obs_t = dev.to_device(obs).reshape(-1)
+    if obs_t.numel() != d:
+        raise ValueError('obs has {} entries, the summaries {} columns'.format(obs_t.numel(), d))
+    W = None
+    if whitening is not None:
+        W = dev.to_device(whitening).contiguous()
+        if tuple(W.shape) != (d, d):
+            raise ValueError('whitening must be a ({0}, {0}) matrix'.format(d))
+    g = None if gammas is None else np.ascontiguousarray(np.atleast_1d(gammas), dtype=np.float64)
+    L = 1 if g is None else len(g)
+    out = dev.empty((P, L))
+    _lib.call('elfi_b200_synlik_f64', dev.context(), SYNLIK_ESTIMATORS[estimator], dev.ptr(S),
+              S.stride(0) if rows > 1 else d, P, n, gs, d, dev.ptr(obs_t), dev.ptr(W), dev.ptr(g),
+              L, dev.ptr(out), dev.stream_ptr())
+    return out
+
+
 def rowsort(x):
     """np.sort(x, axis=1) on the device (ascending, NaN last); order-statistic summaries."""
     x = _matrix(x)

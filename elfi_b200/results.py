@@ -176,3 +176,19 @@ class BolfiSample(Sample):
         outputs = {name: kept[:, i] for i, name in enumerate(parameter_names)}
         super().__init__(method_name=method_name, outputs=outputs, parameter_names=parameter_names,
                          chains=chains, n_chains=chains.shape[0], warmup=warmup, **meta)
+
+
+class BslSample(Sample):
+    """Result of BSL.sample (elfi/methods/results.py:546-605): `samples_all` holds the whole chain
+    (burn-in included), `samples` / `outputs` the draws after burn-in; `acc_rate`, `burn_in` and
+    `n_sim` are attributes."""
+
+    def __init__(self, method_name, samples_all, parameter_names, burn_in=0, acc_rate=None, **meta):
+        outputs = {k: samples_all[k][burn_in:] for k in samples_all}
+        super().__init__(method_name=method_name, outputs=outputs, parameter_names=parameter_names,
+                         samples_all=samples_all, burn_in=burn_in, acc_rate=acc_rate, **meta)
+
+    def compute_ess(self):
+        """Effective sample size of the post-burn-in chain of each parameter."""
+        from .mcmc import eff_sample_size
+        return {p: eff_sample_size(self.samples[p]) for p in self.parameter_names}

@@ -432,6 +432,34 @@ int elfi_b200_kliep_fit_f64(elfi_b200_ctx* ctx, const double* x, int64_t ldx, in
 int elfi_b200_rowsort_f64(elfi_b200_ctx* ctx, const double* X, int64_t ldX, int64_t B, int64_t n,
                           double* out, int64_t ld_out, void* stream);
 
+/* ---- BSL synthetic likelihood (fp64) ----------------------------------------------------------
+ * elfi_b200_synlik_f64: the Gaussian synthetic log-likelihood of P groups of simulated summaries,
+ *   GAUSSIAN      gaussian_syn_likelihood             (elfi/methods/bsl/pdf_methods.py:77-135)
+ *   GHURYE_OLKIN  gaussian_syn_likelihood_ghurye_olkin (elfi/methods/bsl/pdf_methods.py:138-176)
+ * Group g is rows g*group_stride .. g*group_stride + n - 1 of S ((rows, d) row-major, leading
+ * dimension ldS); group_stride > n uses the first n rows of each block (array n_sim of
+ * log_SL_stdev / select_penalty without copies).  Per group: column mean mu and the np.cov
+ * covariance Sigma (ddof 1); with Wh (d x d device, row-major, or NULL) mu' = Wh mu,
+ * Sigma' = Wh Sigma Wh^T, obs' = Wh obs; for each of the L Warton parameters gamma_host[l] (HOST,
+ * in [0, 1]; the reference's cov_warton(Sigma, gamma) = gamma Sigma + (1 - gamma) diag(Sigma_ii +
+ * 1e-5)), a Cholesky factor and
+ *   loglik[g*L + l] = -(|L^-1 (obs - mu)|^2 + log det Sigma + d log 2 pi) / 2.
+ * gamma_host == NULL means no shrinkage (L must be 1).  GHURYE_OLKIN takes neither Wh nor gammas;
+ * its log|det psi| = d log(n-1) + log det Sigma + log|1 - q n / (n-1)^2| with
+ * q = (obs-mu)^T Sigma^-1 (obs-mu) comes from the same factor (sign-blind like the reference's
+ * slogdet).  -inf: a non-finite value in the group, or a pivot <= 1e6 eps max_j A_jj of the
+ * factored matrix A (SciPy's _PSD cutoff constant applied to pivots; this covers n <= d).  A nearly
+ * singular Sigma between that criterion and SciPy's eigenvalue test may be -inf in one
+ * implementation and finite in the other.
+ * Limits: 1 <= d <= ELFI_B200_SYNLIK_MAX_D, n >= 2, group_stride >= n, L >= 1, else ERR_ARG. */
+#define ELFI_B200_SYNLIK_MAX_D 128
+#define ELFI_B200_SYNLIK_GAUSSIAN 0
+#define ELFI_B200_SYNLIK_GHURYE_OLKIN 1
+int elfi_b200_synlik_f64(elfi_b200_ctx* ctx, int32_t estimator, const double* S, int64_t ldS,
+                         int64_t P, int64_t n, int64_t group_stride, int64_t d, const double* obs,
+                         const double* Wh, const double* gamma_host, int64_t L, double* loglik,
+                         void* stream);
+
 #ifdef __cplusplus
 }
 #endif

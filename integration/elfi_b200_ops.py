@@ -6,6 +6,7 @@ buffers and supplies the stream) and plugs into the reference through its own ex
 
     elfi.Distance(device_cdist_euclidean, *summaries)      # elfi/model/elfi_model.py:1016-1019
     elfi.Summary(partial(device_autocov, lag=1), sim)      # elfi/model/elfi_model.py:922-937
+    elfi.BSL(m, n_sim, likelihood=partial(device_gaussian_syn_likelihood, ...))   # bsl.py:35-53
 
 ``tests/test_reference_plugin.py`` runs the reference's own Rejection sampler on a model built
 this way and reproduces the reference's golden result bit for bit.
@@ -71,3 +72,25 @@ def device_autocov(x, lag=1):
         _context(), _P(X.data_ptr()), _I64(n), _I64(B), _I64(n), lags, _I64(1),
         _P(out.data_ptr()), _I64(1), _stream()))
     return out.cpu().numpy()[:, 0]
+
+
+def device_gaussian_syn_likelihood(ssx, ssy, shrinkage=None, penalty=None, whitening=None,
+                                   standardise=False):
+    """Drop-in for elfi.methods.bsl.pdf_methods.gaussian_syn_likelihood (pdf_methods.py:77-135)
+    with shrinkage None or 'warton': ssx (n, d), ssy (d,) or (1, d) -> array([loglik]) from one
+    call of elfi_b200_synlik_f64 (-inf for a singular covariance, like the reference)."""
+    if shrinkage not in (None, 'warton'):
+        raise NotImplementedError('only shrinkage=None or \'warton\' runs on the device')
+    X = _dev(np.atleast_2d(ssx))
+    n, d = X.shape
+    obs = _dev(np.ravel(ssy))
+    Wh = None if whitening is None else _dev(whitening)
+    gam = None
+    if shrinkage == 'warton':
+        gam = (ctypes.c_double * 1)(1 - penalty)
+    out = torch.empty(1, dtype=torch.float64, device='cuda')
+    _check(_lib.elfi_b200_synlik_f64(
+        _context(), ctypes.c_int32(0), _P(X.data_ptr()), _I64(d), _I64(1), _I64(n), _I64(n),
+        _I64(d), _P(obs.data_ptr()), _P(Wh.data_ptr() if Wh is not None else 0), gam, _I64(1),
+        _P(out.data_ptr()), _stream()))
+    return out.cpu().numpy()
